@@ -9,8 +9,10 @@ One "step" = one pass of the hot path over one synthetic 512x512 frame:
 Inputs are resident in HBM for `value`; `e2e` repeats the step through the reference-facing
 drop-in API with pinned host buffers, H2D/D2H inside the timed region.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 Under torchrun (N>1) every rank renders its own frame (weak scaling, no data-path collective).
+--dump-outputs writes what the last timed step computed (rank 0) as DIR/<name>.npy: the inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -151,6 +153,28 @@ def mc_part(sc, eng):
     v, f = MCGpu.mc_gpu(grid[0, 0].permute(2, 1, 0).contiguous(), eng.spacing_x, eng.spacing_y, eng.spacing_z,
                         eng.bx, eng.by, eng.bz, 0.0)
     return grid, v, f
+
+
+DUMP_BUDGET = 60 << 20   # array bytes written by --dump-outputs in all: under 64 MB with the .npy headers
+
+
+def dump_outputs(path, outs, budget=DUMP_BUDGET):
+    """Writes each tensor of `outs` as path/<name>.npy: floating point as float32, integer and bool as float64 (exact
+    for indices).  The budget is shared out smallest tensor first; a tensor larger than its share is replaced by a fixed
+    sample of its elements (flattened, chosen by a seeded permutation of its size, kept in index order), so the same
+    shapes always give the same sample."""
+    os.makedirs(path, exist_ok=True)
+    dtype = lambda t: torch.float32 if t.is_floating_point() else torch.float64
+    order = sorted(outs, key=lambda k: outs[k].numel() * dtype(outs[k]).itemsize)
+    for i, name in enumerate(order):
+        t = outs[name].detach()
+        dt = dtype(t)
+        n = budget // (len(order) - i) // dt.itemsize
+        budget -= min(n, t.numel()) * dt.itemsize
+        if t.numel() > n:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:n].sort()[0]
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.to(dt).cpu().numpy())
 
 
 def layer_roofline(dev, M, launches=24):
@@ -645,7 +669,12 @@ def main():
     ap.add_argument("--impl", default="ours")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-train", action="store_true", help="skip the training-step section")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's results (ray points, convergence mask, colours, SDF grid, "
+                         "mesh) as DIR/<name>.npy, %d MiB at most" % (DUMP_BUDGET >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -691,7 +720,7 @@ def main():
             flush.zero_()
             e0, e1, e2, e3 = ev(), ev(), ev(), ev()
             e0.record()
-            ray_part(sc, rays_d, init_d, bi_d, stats)
+            pts, conv, rgb = ray_part(sc, rays_d, init_d, bi_d, stats)
             e1.record()
             flush.zero_()
             e2.record()
@@ -703,10 +732,13 @@ def main():
         barrier()
         t_wall = time.perf_counter() - t_wall0
     launches = ops.LAUNCHES
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"ray_points": pts, "ray_converged": conv, "ray_rgb": rgb, "sdf_grid": grid,
+                                         "mesh_vertices": v, "mesh_faces": f})
     # second number: weights change every step (a training loop): weight-norm fold + tensor-core weight packing
     # + an eager (not graph-replayed) trace are inside the timed region
     refold_ms = []
-    for _ in range(max(2, args.steps // 2)):
+    for _ in range(args.steps):
         flush.zero_()
         for m in (sc["sdf"], sc["comp"].defs[0], sc["rn"]):
             with torch.no_grad():
@@ -772,7 +804,7 @@ def main():
 
     train = None
     if not args.no_train:
-        train = train_part(sc, dev, rank, world, dist, max(2, min(args.steps, 10)), args.warmup)
+        train = train_part(sc, dev, rank, world, dist, args.steps, args.warmup)
         train_launches = ops.LAUNCHES
         # the scene's parameters moved (Adam): nothing below depends on their values
 
@@ -841,7 +873,7 @@ def main():
     if train is not None:
         wg_ms, wg_flops = wgrad_roofline(dev)
         wg_tf = wg_flops / (wg_ms * 1e-3) / 1e12
-        train["gpu_launches_own_kernels_per_step"] = int(train_launches // max(2, min(args.steps, 10)))
+        train["gpu_launches_own_kernels_per_step"] = int(train_launches // args.steps)
         train["roofline"] = {"kernel": "tc_wgrad_kernel (tcgen05 MN-major split-BF16 GEMM dW = delta^T x, 512x512 over "
                                        "393 216 rows: the def_regu block's translator layers)", "bound": "tensor",
                              "achieved": wg_tf, "peak": pk["tensor"], "unit": "TFLOP/s", "frac": wg_tf / pk["tensor"],

@@ -127,6 +127,16 @@ def elem_err(a, b):
 rel_err = elem_err   # the parity bar of every floating-point test
 
 
+def sha256(a):
+    """Digest of an array's dtype, shape and bytes: a bit-exact comparison against a stored fixture without storing
+    the array itself."""
+    import hashlib
+    a = np.ascontiguousarray(a.detach().cpu().numpy() if torch.is_tensor(a) else a)
+    h = hashlib.sha256(("%s%s" % (a.dtype.str, a.shape)).encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
 def mc_tri_table():
     """The 256x16 triangulation as an int array, decoded from the product's packed table so the
     C oracle and the kernel are checked against one another AND (test_mc_tables) against the

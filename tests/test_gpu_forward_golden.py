@@ -122,9 +122,7 @@ def _run_step(cuda_dev, g, fused):
     from selfreconcode_b200 import train_ops
     net, sdf, comp, rn, cond, cams = _build(cuda_dev, g)
     import utils
-    utils.sample_points = fixed_sample_points
     import model.optim as mo
-    mo.utils.sample_points = fixed_sample_points
     frags = types.SimpleNamespace(pix_to_face=torch.from_numpy(g["pix_to_face"]).to(cuda_dev),
                                   bary_coords=torch.from_numpy(g["bary"]).to(cuda_dev))
     net.raster_seed = lambda dv, tv, tf, cam: frags          # the reference run's own fragments: same seeds
@@ -133,6 +131,9 @@ def _run_step(cuda_dev, g, fused):
     fids = torch.arange(3, device=cuda_dev)
     torch.manual_seed(123)
     train_ops.TC_TRAIN_ENABLED = fused
+    # the stand-in is undone afterwards: later tests in the same process call the real sample_points
+    saved = utils.sample_points, mo.utils.sample_points
+    utils.sample_points = mo.utils.sample_points = fixed_sample_points
     try:
         loss = net.forward(datas, 100000, RATIO, fids)
         info = dict(net.info)
@@ -141,6 +142,7 @@ def _run_step(cuda_dev, g, fused):
         net.propagateTmpPsGrad(fids, RATIO)
     finally:
         train_ops.TC_TRAIN_ENABLED = True
+        utils.sample_points, mo.utils.sample_points = saved
     named = [("sdf." + k, q) for k, q in sorted(sdf.named_parameters())] + \
             [("def." + k, q) for k, q in sorted(comp.named_parameters())] + \
             [("rn." + k, q) for k, q in sorted(rn.named_parameters())] + list(zip(("poses", "trans", "dcond"), cond))

@@ -3,7 +3,8 @@
 Every test calls the product through its C-ABI wrappers / drop-in modules and compares with
   (1) the golden vectors recorded from the unmodified reference (tests/golden/),
   (2) the CPU oracle on the same seeded inputs,
-  (3) where built, the reference's own CUDA kernels from oracle/_ref/ (A/B on the same GPU).
+  (3) the outputs of the reference's own CUDA kernels on the same seeded inputs, recorded on a B200
+      (tests/golden/ref_kernels.npz, written by oracle/make_golden_ref.py).
 Bars: bit-exact for integer / index work (MC faces and vertex ids, sampler corner indices,
 masks away from thresholds, boundary flags); 1e-4 norm-wise relative for floating point
 (the north star's tolerance), tighter where the arithmetic allows it.
@@ -14,7 +15,7 @@ import torch
 
 from helpers import (RATIO, SMPL_PARENTS, build_render, build_sdf_full, build_sdf_small,
                      build_skinner, build_translator, dropin, golden, mc_tri_table, plain_params,
-                     norm_err, rel_err, sdf_params, wn_params)
+                     norm_err, rel_err, sdf_params, sha256, wn_params)
 
 pytestmark = pytest.mark.gpu
 FP_TOL = 1e-4
@@ -25,9 +26,34 @@ def helpers_root():
     return helpers.ROOT
 
 
-def _ref(name):
-    from oracle import build
-    return build.load_ref(name)
+def _sampled(g, key):
+    """(flat indices, values) of a reference output stored as a seeded sample of its elements."""
+    return g[key + "_idx"], g[key + "_val"]
+
+
+# Inputs of the comparisons with the reference's CUDA kernels (oracle/make_golden_ref.py runs the same functions).
+def _minv_ab_inputs():
+    """50 000 matrices; the backward kernel is compared on 512 of them (`rows`) with gradients `gr`."""
+    ms = torch.randn(50000, 3, 3, generator=torch.Generator().manual_seed(1))
+    rows = torch.randperm(ms.shape[0], generator=torch.Generator().manual_seed(2))[:512].sort()[0]
+    gr = torch.randn(512, 3, 3, generator=torch.Generator().manual_seed(3))
+    return ms, rows, gr
+
+
+def _interp_ab_inputs():
+    g = torch.Generator().manual_seed(6)
+    x = torch.randn(1, 1, 33, 41, 17, generator=g)
+    y = torch.randn(1, 1, 65, 81, 33, generator=g)      # output gradient for the backward kernel
+    return x, y
+
+
+def _grid_sampler_ab_inputs():
+    g = torch.Generator().manual_seed(5)
+    inp = torch.rand(1, 24, 9, 17, 11, generator=g)
+    grid = (torch.rand(1, 1, 1, 3000, 3, generator=g) - 0.5) * 2.2
+    go = torch.randn(1, 24, 1, 1, 3000, generator=g)
+    ggi, ggg = torch.randn(inp.shape, generator=g), torch.randn(grid.shape, generator=g)
+    return inp, grid, go, ggi, ggg
 
 
 # ------------------------------------------------------------------------------------------------
@@ -72,32 +98,34 @@ def test_minv3x3_forward_backward(cuda_dev):
     assert inv0.shape == (0, 3, 3) and chk0.shape == (0,)
 
 
+def _minv_adjugate_err(inv, ms, ok):
+    """rel_err of inverse * |det| * sign(det) against the float64 adjugate over the invertible rows `ok`."""
+    det = torch.linalg.det(ms.double()).view(-1, 1, 1)
+    adj = (torch.linalg.inv(ms.double()) * det).cpu().numpy()
+    return rel_err((inv.double() * det.abs() * torch.sign(det)).cpu().numpy()[ok], adj[ok])
+
+
 def test_minv3x3_matches_reference_kernel(cuda_dev):
-    ref = _ref("FastMinv")
-    if ref is None:
-        pytest.skip("oracle/_ref/FastMinv.so not built")
+    ref = golden("ref_kernels.npz")
     dropin()
     import FastMinv
-    ms = torch.randn(50000, 3, 3, generator=torch.Generator().manual_seed(1)).to(cuda_dev)
+    ms, _, gr = _minv_ab_inputs()
+    ms = ms.to(cuda_dev)
     a, ac = FastMinv.Fast3x3Minv(ms)
-    b, bc = ref.Fast3x3Minv(ms)
     torch.cuda.synchronize()
-    assert torch.equal(ac, bc), "singularity mask identical to the reference kernel"
-    det = torch.linalg.det(ms.double()).abs().view(-1, 1, 1)
+    bc = np.unpackbits(ref["minv_mask"])[:ms.shape[0]].astype(bool)
+    assert np.array_equal(ac.cpu().numpy(), bc), "singularity mask identical to the reference kernel"
     # floating point: the 2x2 minors cancel, and FMA contraction differs between the two builds, so
     # the two kernels agree to the conditioning of the minors, not to the last bit: both must be
-    # equally close to the float64 adjugate.
-    adj = (torch.linalg.inv(ms.double()) * torch.linalg.det(ms.double()).view(-1, 1, 1)).cpu().numpy()
-    sgn = torch.sign(torch.linalg.det(ms.double())).view(-1, 1, 1)
+    # equally close to the float64 adjugate (the reference kernel's distance is stored).
     m = ac.cpu().numpy()  # invertible ones (the others are zeroed by both kernels)
-    assert (a[~ac] == 0).all() and (b[~bc] == 0).all()
-    ea = rel_err((a.double() * det * sgn).cpu().numpy()[m], adj[m])
-    eb = rel_err((b.double() * det * sgn).cpu().numpy()[m], adj[m])
+    assert (a[~ac] == 0).all()
+    ea = _minv_adjugate_err(a, ms, m)
+    eb = float(ref["minv_adj_err"])
     assert ea < 5e-4 and eb < 5e-4 and ea < 2 * eb + 1e-6
-    gr = torch.randn_like(ms)
-    # same inputs to both backward kernels (the inverses above differ in the last bits)
-    assert rel_err(FastMinv.Fast3x3Minv_backward(gr, a).cpu().numpy(),
-                   ref.Fast3x3Minv_backward(gr, a).cpu().numpy()) < 1e-6
+    # same inputs to both backward kernels: the reference kernel's inverses of 512 of the matrices
+    bo = FastMinv.Fast3x3Minv_backward(gr.to(cuda_dev), torch.from_numpy(ref["minv_bwd_inv"]).to(cuda_dev))
+    assert rel_err(bo.cpu().numpy(), ref["minv_bwd"]) < 1e-6
 
 
 # ------------------------------------------------------------------------------------------------
@@ -163,23 +191,21 @@ def _canon(v, f):
     return v[order], f2
 
 
+MC_AB_CASES = ((33, True), (129, False))
+MC_AB_ARGS = (0.0078125, 0.0078125, 0.0078125, -1.0, -1.0, -1.0, 0.0)
+
+
 def test_mc_matches_reference_kernel(cuda_dev):
-    ref = _ref("MCGpu")
-    if ref is None:
-        pytest.skip("oracle/_ref/MCGpu.so not built")
+    ref = golden("ref_kernels.npz")
     dropin()
     import MCGpu
-    for n, aniso in ((33, True), (129, False)):
+    for n, aniso in MC_AB_CASES:
         grid = _test_grid(n, 100 + n, aniso).to(cuda_dev)
-        args = (0.0078125, 0.0078125, 0.0078125, -1.0, -1.0, -1.0, 0.0)
-        v, f = MCGpu.mc_gpu(grid, *args)
-        rv, rf = ref.mc_gpu(grid, *args)
-        torch.cuda.synchronize()
-        assert v.shape == rv.shape and f.shape == rf.shape
+        v, f = MCGpu.mc_gpu(grid, *MC_AB_ARGS)
+        assert (v.shape[0], f.shape[0]) == (int(ref["mc%d_nv" % n]), int(ref["mc%d_nf" % n]))
         cv, cf = _canon(v.cpu().numpy(), f.cpu().numpy())
-        rcv, rcf = _canon(rv.cpu().numpy(), rf.cpu().numpy())
-        assert np.array_equal(cv, rcv), "vertex positions bit-identical to the reference kernel"
-        assert np.array_equal(cf, rcf), "faces identical after canonicalising the race-ordered ids"
+        assert sha256(cv) == ref["mc%d_v_sha" % n], "vertex positions bit-identical to the reference kernel"
+        assert sha256(cf) == ref["mc%d_f_sha" % n], "faces identical after canonicalising the race-ordered ids"
 
 
 def test_mc_full_size_properties(cuda_dev):
@@ -222,15 +248,13 @@ def test_interp2x3d(cuda_dev):
         y = torch.randn(out.shape, generator=g).to(cuda_dev)
         gin = op.backward(y)
         assert abs((out * y).sum().item() - (x.to(cuda_dev) * gin).sum().item()) < 1e-3 * max(1.0, out.numel() ** 0.5)
-    r = _ref("interp2x_boundary3d")
-    if r is not None:
-        x = torch.randn(1, 1, 33, 41, 17, generator=g).to(cuda_dev)
-        a, ab = op.forward(x, 0.0)
-        b, bb = r.forward(x, 0.0)
-        torch.cuda.synchronize()
-        assert torch.equal(a, b) and torch.equal(ab, bb)
-        y = torch.randn_like(a)
-        assert torch.allclose(op.backward(y), r.backward(y), atol=1e-6)
+    # against the reference kernel
+    ref = golden("ref_kernels.npz")
+    x, y = _interp_ab_inputs()
+    a, ab = op.forward(x.to(cuda_dev), 0.0)
+    assert sha256(a) == ref["i2x_out_sha"] and sha256(ab) == ref["i2x_bnd_sha"]
+    idx, want = _sampled(ref, "i2x_bwd")
+    assert np.allclose(op.backward(y.to(cuda_dev)).cpu().numpy().reshape(-1)[idx], want, rtol=1e-5, atol=1e-6)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -268,24 +292,22 @@ def test_grid_sampler_gradcheck_first_and_second_order(cuda_dev):
 
 
 def test_grid_sampler_matches_reference_kernels(cuda_dev):
-    r = _ref("GridSamplerMine")
-    if r is None:
-        pytest.skip("oracle/_ref/GridSamplerMine.so not built")
+    ref = golden("ref_kernels.npz")
     dropin()
     import GridSamplerMine as op
-    g = torch.Generator().manual_seed(5)
-    inp = torch.rand(1, 24, 9, 17, 11, generator=g).to(cuda_dev)
-    grid = ((torch.rand(1, 1, 1, 3000, 3, generator=g) - 0.5) * 2.2).to(cuda_dev)
-    a, b = op.forward(inp, grid, 0, 1), r.forward(inp, grid, 0, 1)
-    assert torch.equal(a, b), "forward bit-identical to the reference kernel"
-    go = torch.randn_like(a)
-    (gi, gg), (ri, rg) = op.backward(inp, grid, go, 0, 1), r.backward(inp, grid, go, 0, 1)
-    assert torch.allclose(gi, ri, atol=1e-5) and torch.allclose(gg, rg, atol=2e-4, rtol=1e-4)
-    ggi, ggg = torch.randn_like(inp), torch.randn_like(grid)
+    inp, grid, go, ggi, ggg = [t.to(cuda_dev) for t in _grid_sampler_ab_inputs()]
+    a = op.forward(inp, grid, 0, 1)
+    assert sha256(a) == ref["gs_fwd_sha"], "forward bit-identical to the reference kernel"
+    gi, gg = op.backward(inp, grid, go, 0, 1)
+    for x, key, atol, rtol in ((gi, "gs_gi", 1e-5, 1e-5), (gg, "gs_gg", 2e-4, 1e-4)):
+        idx, want = _sampled(ref, key)
+        assert np.allclose(x.cpu().numpy().reshape(-1)[idx], want, rtol=rtol, atol=atol), key
     o = op.dbackward(ggi, ggg, inp, grid, go, 0, 1)
-    ro = r.dbackward(ggi, ggg, inp, grid, go, 0, 1)
-    for x, y in zip(o, ro):
-        assert rel_err(x.cpu().numpy(), y.cpu().numpy()) < 1e-4
+    for i, x in enumerate(o):
+        # rel_err's floor (mean |reference|) is taken over the whole reference output
+        idx, want = _sampled(ref, "gs_dd%d" % i)
+        err = np.abs(x.cpu().numpy().reshape(-1)[idx].astype(np.float64) - want) / (np.abs(want) + ref["gs_dd%d_absmean" % i])
+        assert err.max() < 1e-4, i
 
 
 # ------------------------------------------------------------------------------------------------
